@@ -1,12 +1,14 @@
 #!/usr/bin/env python
 """bench.py -- BFV ct x ct mul+relinearize throughput at N=2^15, 14x62-bit q (BASELINE.json).
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--batch B]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--batch B] [--dump-outputs DIR]
 
 A "step" is one pass of Multiplicator::multiply over one batch of `--batch` ciphertext pairs
 per GPU (synthetic uniform residues, as fresh BFV ciphertext halves are).  Prints ONE JSON line
 (rank 0).  `--impl reference` times the reference's CPU algorithm instead (the oracle port --
 the Rust reference cannot be built in this image), on all host cores, same metric/config.
+`--dump-outputs DIR` writes a fixed sample of rank 0's products of the last timed step to DIR
+(see dump_outputs); the inputs depend only on the arguments, so two builds can be compared file by file.
 """
 from __future__ import annotations
 
@@ -208,6 +210,29 @@ def verify_against_oracle(np, A, Bt, out, rot, kc, gc, indices):
     return ok_mul, ok_rot
 
 
+def dump_outputs(np, out, directory, n_ct=16, n_coeff=2048):
+    """Writes a fixed sample of the product batch `out` as float64 .npy files (about 15 MB):
+      products.npy            [n_ct][2][N_MODULI][n_coeff][2]  each u64 residue as (high 32 bits, low 32 bits),
+                                                               both exact in float64
+      ciphertext_index.npy    [n_ct]     which ciphertexts of the batch (always the first, the last and both sides of
+                                         the library's 256-ciphertext chunk boundary)
+      coefficient_index.npy   [n_coeff]  which coefficients of every polynomial
+    The sample is drawn from a fixed seed, so it is the same for every run with the same --batch."""
+    count = out.shape()[0]
+    rng = np.random.default_rng(12345)
+    fixed = sorted(set(i for i in (0, 255, 256, count - 1) if i < count))
+    rest = np.setdiff1d(np.arange(count), fixed)
+    cts = np.sort(np.concatenate([fixed, rng.choice(rest, min(len(rest), n_ct - len(fixed)), replace=False)]))
+    coeffs = np.sort(rng.choice(DEGREE, n_coeff, replace=False))
+    one = np.empty((1, 2, N_MODULI, DEGREE), np.uint64)
+    words = np.stack([out.to_host(one, first=int(i))[0][:, :, coeffs] for i in cts])
+    split = np.stack([words >> np.uint64(32), words & np.uint64(0xFFFFFFFF)], axis=-1).astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "products.npy"), split)
+    np.save(os.path.join(directory, "ciphertext_index.npy"), cts.astype(np.float64))
+    np.save(os.path.join(directory, "coefficient_index.npy"), coeffs.astype(np.float64))
+
+
 def cpu_baseline_sample():
     """single-thread oracle port on a bounded sample (3 products at the full size)"""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
@@ -247,7 +272,12 @@ def main():
     # 1024 -> 3440 products/s on one B200 (copy-only ceiling 3550).  512 keeps the pinned staging at 11 GB per rank.
     ap.add_argument("--e2e-batch", type=int, default=int(os.environ.get("FHE_BENCH_E2E_BATCH", "512")))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a sample of the last timed step's products to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the products of the GPU path only")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -346,6 +376,8 @@ def main():
     n_out_words = B * 2 * N_MODULI * DEGREE
     cs = int(torch.as_tensor(DevArray(out.device_ptr(), n_out_words), device="cuda").sum().item()) & ((1 << 63) - 1)
     checksums = gather_checksums([cs], device="cuda")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(np, out, args.dump_outputs)
 
     # ct + ct (the HBM-bound member of the family): rot += out, 3 rows of traffic per limb row
     for _ in range(2):

@@ -42,10 +42,9 @@ def test_shard_range_properties():
 def test_two_rank_gloo(tmp_path):
     script = tmp_path / "worker.py"
     script.write_text(WORKER)
-    env = dict(os.environ, MASTER_ADDR="127.0.0.1", MASTER_PORT="29541")
-    out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
-                          "--master-addr", "127.0.0.1", "--master-port", "29541", str(script), ROOT],
-                         capture_output=True, text=True, timeout=300, env=env)
+    # --standalone: a local rendezvous on a free port, so that concurrent runs on one host do not collide
+    out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--standalone", "--nproc-per-node=2",
+                          str(script), ROOT], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0 and "SHARD_OK" in out.stdout, out.stdout + out.stderr
 
 
